@@ -4,11 +4,14 @@
     python bench.py --gpus 1 --steps K --warmup W            # our arm, one B200
     torchrun ... bench.py --gpus N --steps K --warmup W      # N ranks, one per GPU
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   # also save what the timed steps computed, DIR/<name>.npy
 
 Headline (the JSON line's own keys): a "step" is one forward of the hot path over one batch of 64 synthetic utterances
 (64 fbank x 160 frames -> 512-d), BASELINE.json configs[1]; N ranks = N utterance-sharded replicas, no collective.
-The K-step timed window is repeated (5..50 windows, >= 0.5 s of device time in total) and the MEDIAN window is
-reported (`windows` holds the spread), so the driver's 20-step runs are not 4-ms single samples.
+Every workload runs W untimed warm-up steps, then ONE timed window of exactly K steps (CUDA events, max over ranks),
+which opens once the host has queued its first steps (see hold()).
+All inputs and weights come from fixed seeds, so the same arguments give the same inputs in every run, and the outputs
+saved by --dump-outputs can be compared between two builds.
 
 Sub-records of the same line (default --workload all):
   "train"    : the triplet training step of BASELINE configs[2] (N=1) / configs[4] (N=8: data parallel, ONE NCCL
@@ -26,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "speaker-embeddings/sec (64-fbank x 160-frame -> 512-d)"
 FLOP_PER_EMB = 2306670592            # BASELINE.md §2 (forward)
@@ -159,7 +163,7 @@ def pick_cpu_threads(sd, T):
 
 
 def cpu_forward_timer(sd, B, T, budget_s, threads):
-    """Times the oracle's eval forward (restatement of /root/reference/model.py:185-218) on host cores."""
+    """Times the oracle's eval forward (restatement of the reference's model.py:185-218) on host cores."""
     import torch
 
     from oracle import rescnn_oracle as O
@@ -181,7 +185,7 @@ def cpu_forward_timer(sd, B, T, budget_s, threads):
 
 
 def workload_config(args, world, dtype_note=True):
-    """The `config` object of the JSON line: identical for our arm and the reference arm (the driver compares them)."""
+    """The `config` object of the JSON line: identical for our arm and the reference arm, so the two lines compare."""
     B, T = args.batch, args.frames
     in_bytes = B * T * 64 * 4
     nbuf = L2_BYTES // in_bytes + 8
@@ -193,8 +197,8 @@ def workload_config(args, world, dtype_note=True):
 
 
 def run_reference(args, rank, world):
-    """--impl reference: the reference's own CPU implementation of the path.  /root/reference does not exist
-    on the GPU box, so this runs the oracle port (same PyTorch CPU kernels the reference dispatches to)."""
+    """--impl reference: the reference's CPU implementation of the path, run as the oracle port (the same PyTorch
+    CPU kernels the reference dispatches to), so that no copy of the reference is needed."""
     if rank != 0:
         return
     import torch
@@ -235,12 +239,6 @@ def run_reference(args, rank, world):
     emit(line)
 
 
-def median(v):
-    s = sorted(v)
-    n = len(s)
-    return s[n // 2] if n % 2 else 0.5 * (s[n // 2 - 1] + s[n // 2])
-
-
 class Dist:
     """Rank / world plumbing shared by the three workloads (torch.distributed over NCCL when world > 1)."""
 
@@ -270,17 +268,43 @@ class Dist:
         return t.tolist()
 
 
-def timed_windows(D, window, K, min_total_ms=500.0, r_min=5, r_max=50):
-    """Repeats the K-step timed window (each bracketed by barrier + synchronize on both sides, CUDA events on the
-    launching stream) until at least `min_total_ms` of device time has been measured (5..50 windows): a 20-step window
-    of a 0.2 ms step lasts 4 ms, too short for one sample to be trusted or for nvidia-smi to see the load.  Returns the
-    per-window milliseconds, max over ranks window by window."""
-    times = [window()]
-    pilot = D.max_over_ranks(times)[0]
-    R = int(min(r_max, max(r_min, -(-min_total_ms // max(pilot, 1e-3)))))
-    for _ in range(R - 1):
-        times.append(window())
-    return D.max_over_ranks(times)
+def timed_window(D, window):
+    """Runs the timed window once: exactly --steps steps, bracketed by barrier + synchronize on both sides, CUDA events
+    on the launching stream.  Returns its milliseconds, the max over ranks."""
+    return D.max_over_ranks([window()])[0]
+
+
+HOLD_CYCLES = 20_000_000    # ~10 ms at the B200's 1965 MHz boost clock
+
+
+def hold(stream):
+    """Called between a window's opening synchronize and its first event: keeps `stream` busy for ~10 ms (one spinning
+    thread) so that the host has queued the window's first steps before they can start.  Every stream of a step orders
+    after the launching stream, so the window times the steps back to back.  A 20-step inference window lasts 3.6 ms, and
+    without the hold it also timed any delay of the host thread while it queued them: on a B200 (1000 W limit) single
+    windows then ranged from 33 k to 353 k emb/s, with it 353.1 k to 353.7 k."""
+    import torch
+
+    with torch.cuda.stream(stream):
+        torch.cuda._sleep(HOLD_CYCLES)
+
+
+DUMP_MAX_ELEMS = 1 << 20    # per array (4 MB in fp32, 8 MB in fp64): the seven arrays of a run stay well below 64 MB in all
+
+
+def write_outputs(out_dir, outputs):
+    """--dump-outputs: one DIR/<name>.npy per array of what the timed steps computed in their last step, float32 (float64
+    for integer results, which it holds exactly).  An array above DUMP_MAX_ELEMS is replaced by a fixed, seeded sample of
+    its flattened elements, so two runs with the same arguments sample the same positions."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def conv_kernel_hash():
@@ -309,8 +333,9 @@ def measured_traffic(B, T):
     return None, f"no ncu capture recorded for kernel build {key} at batch {B}"
 
 
-def bench_infer(args, D):
-    """The headline: batch-64 eval inference (BASELINE configs[1]) through EmbeddingPipeline."""
+def bench_infer(args, D, outputs):
+    """The headline: batch-64 eval inference (BASELINE configs[1]) through EmbeddingPipeline.  Puts the embeddings of
+    the last timed step into `outputs`."""
     import ctypes
 
     import torch
@@ -330,6 +355,7 @@ def bench_infer(args, D):
     cur = torch.cuda.current_stream(dev)
     cnt = [0]
     host_ms = []
+    last = [None]
     with torch.no_grad():
         sampler = ClockSampler(D.local_rank)
         if rank == 0:
@@ -339,6 +365,10 @@ def bench_infer(args, D):
         for i in range(2 * args.lanes):
             pipe.embed_device(xs[i % nbuf])
         pipe.synchronize()
+        # the clock samples start here, and the warm-up steps follow at once: no idle gap before the timed window
+        D.barrier()
+        if rank == 0:
+            sampler.mark()
         for i in range(W):
             pipe.embed_device(xs[i % nbuf])
         pipe.synchronize()
@@ -346,10 +376,11 @@ def bench_infer(args, D):
         # ---- value: inputs resident in HBM; `lanes` forwards in flight through the public pipeline ------------------
         def window():
             D.barrier()
+            hold(cur)
             e0.record(cur)
             t_host = time.perf_counter()
             for _ in range(K):
-                pipe.embed_device(xs[cnt[0] % nbuf])
+                last[0] = pipe.embed_device(xs[cnt[0] % nbuf])
                 cnt[0] += 1
             host_ms.append((time.perf_counter() - t_host) * 1e3 / K)
             for st in pipe.lanes:
@@ -358,18 +389,20 @@ def bench_infer(args, D):
             D.barrier()
             return e0.elapsed_time(e1)
 
-        D.barrier()
-        if rank == 0:
-            sampler.mark()
-        ws = timed_windows(D, window, K)
-        ms = median(ws)
+        ms = timed_window(D, window)
         value = world * B * K / (ms * 1e-3)
-        host_ms_value = median(host_ms)
+        host_ms_value = host_ms[0]
+        outputs["embeddings"] = last[0].cpu().numpy()
 
         # ---- e2e: host buffers through the public API, H2D + D2H inside the timed region -----------
         nhost = 8
         xh = [torch.randn(B, 1, T, 64).pin_memory() for _ in range(nhost)]
         oh = [torch.empty(B, 512).pin_memory() for _ in range(nhost)]
+        # one-time setup outside the W warm-up steps: the pipeline allocates the device buffers of each of its
+        # lanes x depth staging slots at the slot's first use, so every slot is used once before the timed window
+        for i in range(len(pipe.lanes) * pipe.depth):
+            pipe.embed(xh[i % nhost], oh[i % nhost])
+        pipe.synchronize()
         for i in range(W):
             pipe.embed(xh[i % nhost], oh[i % nhost])
         pipe.synchronize()
@@ -377,6 +410,7 @@ def bench_infer(args, D):
 
         def window_e2e():
             D.barrier()
+            hold(pipe.h2d)
             e0.record(pipe.h2d)
             t_host = time.perf_counter()
             for _ in range(K):
@@ -388,11 +422,10 @@ def bench_infer(args, D):
             D.barrier()
             return e0.elapsed_time(e1)
 
-        ws2 = timed_windows(D, window_e2e, K)
+        ms_e2e = timed_window(D, window_e2e)
         clocks = sampler.stop() if rank == 0 else None
-        ms_e2e = median(ws2)
         e2e_value = world * B * K / (ms_e2e * 1e-3)
-        host_ms_e2e = median(host_ms2)
+        host_ms_e2e = host_ms2[0]
 
         # ---- roofline of the dominant kernel: per-launch CUDA-event times inside the forward ---------
         eng = model._engine
@@ -450,7 +483,7 @@ def bench_infer(args, D):
         cpu_baseline = {"value": v, "unit": "emb/s", "cores": threads, "host_cpus": os.cpu_count(),
                         "kind": "port",
                         "sample": f"{n_it} forwards of the same batch-{B} workload in {el:.1f} s (oracle port of "
-                                  f"/root/reference/model.py:185-218, torch CPU fp32)"}
+                                  f"model.py:185-218, torch CPU fp32)"}
     cfg = workload_config(args, world)
     line = {
         "metric": METRIC, "value": value, "unit": "emb/s", "n_gpus": world, "steps": K, "warmup": W,
@@ -459,10 +492,9 @@ def bench_infer(args, D):
         "engine": {"forwards_in_flight": args.lanes,
                    "operands": f"{args.dtype} tensor-core operands (BASELINE names bf16: same width and tensor-pipe rate; bf16 "
                                f"misses the 1e-3 parity bar, --dtype bf16 runs it), fp32 accumulate/BN/fc/norm"},
-        "windows": {"n": len(ws), "timing": "median of n windows of exactly `steps` steps, each bracketed by barrier + "
-                                            "synchronize, CUDA events, max over ranks per window",
-                    "ms_per_step_min": min(ws) / K, "ms_per_step_max": max(ws) / K,
-                    "e2e_n": len(ws2), "e2e_ms_per_step_min": min(ws2) / K, "e2e_ms_per_step_max": max(ws2) / K},
+        "timing": "one window of exactly `steps` steps after `warmup` untimed steps, bracketed by barrier + synchronize, "
+                  "CUDA events, max over ranks; the launching stream is held ~10 ms before the first event so that the "
+                  "first steps are queued when the window opens",
         "clocks": clocks,
         "host_enqueue_ms_per_step": host_ms_value,
         "e2e": {"value": e2e_value, "unit": "emb/s", "h2d_bytes_per_step": in_bytes, "d2h_bytes_per_step": B * 512 * 4,
@@ -477,10 +509,10 @@ def bench_infer(args, D):
     return line
 
 
-def bench_other_dtype(args, D):
+def bench_other_dtype(args, D, outputs):
     """The same headline workload with the OTHER 16-bit operand format (bf16 when the line is fp16): BASELINE names bf16,
     the engine defaults to fp16 because bf16 misses the 1e-3 parity bar (DESIGN.md §2); both run at the same tensor-pipe
-    rate, and this record keeps the bf16 number beside the headline.  value only (inputs resident), same windows."""
+    rate, and this record keeps the bf16 number beside the headline.  value only (inputs resident), same timing."""
     import torch
 
     from deepspeaker_pytorch_b200 import EmbeddingPipeline
@@ -495,16 +527,18 @@ def bench_other_dtype(args, D):
     cur = torch.cuda.current_stream(dev)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     cnt = [0]
+    last = [None]
     with torch.no_grad():
-        for i in range(2 * args.lanes + max(args.warmup, 3)):
+        for i in range(2 * args.lanes + args.warmup):
             pipe.embed_device(xs[i % nbuf])
         pipe.synchronize()
 
         def window():
             D.barrier()
+            hold(cur)
             e0.record(cur)
             for _ in range(K):
-                pipe.embed_device(xs[cnt[0] % nbuf])
+                last[0] = pipe.embed_device(xs[cnt[0] % nbuf])
                 cnt[0] += 1
             for st in pipe.lanes:
                 cur.wait_stream(st)
@@ -512,13 +546,13 @@ def bench_other_dtype(args, D):
             D.barrier()
             return e0.elapsed_time(e1)
 
-        ws = timed_windows(D, window, K, min_total_ms=200.0, r_min=5, r_max=25)
-    ms = median(ws)
-    return {"dtype": other, "value": D.world * B * K / (ms * 1e-3), "unit": "emb/s", "ms_per_step": ms / K, "windows": len(ws),
+        ms = timed_window(D, window)
+    outputs["other_dtype_embeddings"] = last[0].cpu().numpy()
+    return {"dtype": other, "value": D.world * B * K / (ms * 1e-3), "unit": "emb/s", "ms_per_step": ms / K, "steps": K,
             "parity": "eval embeddings ~3e-3 vs the fp32 reference (bar 1e-3)" if other == "bf16" else "eval embeddings 4e-4 - 7e-4 (bar 1e-3)"}
 
 
-def bench_allpairs(args, D):
+def bench_allpairs(args, D, outputs):
     """BASELINE configs[3]: 1024-utterance all-pairs distance matrix + top-8 hard-negative select (single GPU,
     launch-latency bound: reported in microseconds).  No reference implementation exists (SURVEY §0 fact 3); the
     CPU figure beside it is the oracle's C restatement (oracle/dsk_oracle.c) on one core."""
@@ -534,28 +568,30 @@ def bench_allpairs(args, D):
         E = torch.randn(N, Dm, device=dev, generator=g)
         sets.append(10.0 * E / E.norm(dim=1, keepdim=True))
     labels = (torch.arange(N, device=dev) // 16).long()
-    K, W = max(20, min(args.steps, 200)), max(3, args.warmup)
+    K, W = args.steps, args.warmup
     for i in range(W):
         allpairs_topk(sets[i % 8], labels, k)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last = [None]
 
     def window():
         torch.cuda.synchronize()
+        hold(torch.cuda.current_stream())
         e0.record()
         for i in range(K):
-            allpairs_topk(sets[i % 8], labels, k)
+            last[0] = allpairs_topk(sets[i % 8], labels, k)
         e1.record()
         torch.cuda.synchronize()
         return e0.elapsed_time(e1)
 
-    ws = [window() for _ in range(5)]
-    us = median(ws) / K * 1e3
+    us = window() / K * 1e3
+    outputs["allpairs_idx"], outputs["allpairs_val"] = (t.cpu().numpy() for t in last[0])
     # algorithmic bytes: read E (N x D fp32) + labels, write idx (int64) + val (fp32); flops: N*N*D MACs of the Gram
     alg_bytes = N * Dm * 4 + N * 8 + N * k * 12
     peaks = load_peaks()
     rec = {"metric": "microseconds per 1024-utterance all-pairs distance + top-8 select", "value": us, "unit": "us",
-           "steps": K, "warmup": W, "windows": len(ws), "higher_is_better": False, "dtype": "f32 (fp16 tensor-core Gram + exact fp32 refinement)",
+           "steps": K, "warmup": W, "higher_is_better": False, "dtype": "f32 (fp16 tensor-core Gram + exact fp32 refinement)",
            "config": {"workload": "1024 x 512 embeddings (norm 10), 64 speakers x 16, k=8, different-speaker candidates "
                                   "(BASELINE configs[3])", "result": "bit-identical indices and distances to the all-fp32 path and the C oracle"},
            "gflops": 2.0 * N * N * Dm / (us * 1e-6) / 1e9,
@@ -586,7 +622,7 @@ def bench_allpairs(args, D):
 TRAIN_FLOP_PER_UTT = 6911819776     # BASELINE.md §2 (forward + backward)
 
 
-def bench_train(args, D):
+def bench_train(args, D, outputs):
     """BASELINE configs[2] (N=1) / configs[4] (N=8): triplet training step restating train_triplet.py:215-224 with the
     drop-in classes — three train-mode forwards of 128 utterances (issued together through forward_triplet: identical
     results, the three calls and their backwards overlap on three streams), TripletMarginLoss, backward, ONE gradient
@@ -598,8 +634,7 @@ def bench_train(args, D):
 
     dev, world, rank = D.dev, D.world, D.rank
     B, T = 128, args.frames
-    K = max(3, min(args.steps, 10))
-    W = 3
+    K, W = args.steps, args.warmup
     model = make_model(args.dtype, dev).train()
     broadcast_parameters(model)
     opt = FusedAdagrad(path_parameters(model), lr=0.1, lr_decay=1e-4, weight_decay=0.0)   # train_triplet.py:70-77,378-382
@@ -615,7 +650,7 @@ def bench_train(args, D):
         loss.backward()                                             # :223
         opt.allreduce()                                             # the one collective of the step
         opt.step()                                                  # :224
-        return loss
+        return loss, (out_a, out_p, out_n)
 
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for i in range(W):
@@ -624,6 +659,7 @@ def bench_train(args, D):
 
     def window():
         D.barrier()
+        hold(torch.cuda.current_stream(dev))
         e0.record()
         for _ in range(K):
             last[0] = step(*xs[cnt[0] % nset])
@@ -633,9 +669,16 @@ def bench_train(args, D):
         return e0.elapsed_time(e1)
 
     last = [None]
-    ws = timed_windows(D, window, K, min_total_ms=600.0, r_min=7, r_max=9)
-    ms = median(ws) / K
-    loss_value = float(last[0].item())    # loss of the last timed step (48 distinct batches: no memorisation)
+    ms = timed_window(D, window) / K
+    loss, outs = last[0]
+    loss_value = float(loss.item())    # loss of the last timed step (48 distinct batches: no memorisation)
+    # what the step hands back (loss, the three embedding batches) and what it changed: the updated parameters, as a fixed
+    # sample of the flat trained parameters
+    flat = torch.cat([p.detach().reshape(-1) for p in path_parameters(model)])
+    pick = torch.randint(flat.numel(), (1 << 16,), generator=torch.Generator().manual_seed(0)).to(dev)
+    outputs["train_loss"] = loss.detach().reshape(1).cpu().numpy()
+    outputs["train_embeddings"] = torch.stack([o.detach() for o in outs]).cpu().numpy()
+    outputs["train_params_sample"] = flat[pick].cpu().numpy()
     # e2e: pinned host inputs copied in (on a copy stream, one batch ahead of the step that consumes it - the prefetch any
     # input pipeline does; every step's 15.7 MB still crosses PCIe inside the timed region), loss read back, every step
     nh = 4
@@ -656,6 +699,7 @@ def bench_train(args, D):
 
     def window_e2e():
         D.barrier()
+        hold(cur)
         for ev in freed:
             ev.record(cur)
         e0.record()
@@ -665,7 +709,7 @@ def bench_train(args, D):
             if j + 1 < K:
                 stage((j + 1) % 2, cnt[0] + 1)
             cur.wait_event(ready[slot])
-            loss = step(*xd[slot])
+            loss, _ = step(*xd[slot])
             freed[slot].record(cur)
             lh.copy_(loss.detach().reshape(1), non_blocking=True)
             cnt[0] += 1
@@ -673,8 +717,7 @@ def bench_train(args, D):
         D.barrier()
         return e0.elapsed_time(e1)
 
-    ws2 = timed_windows(D, window_e2e, K, min_total_ms=300.0, r_min=3, r_max=5)
-    ms2 = median(ws2) / K
+    ms2 = timed_window(D, window_e2e) / K
     if rank != 0:
         return None
     peaks = load_peaks()
@@ -682,9 +725,7 @@ def bench_train(args, D):
     achieved = 3 * B * TRAIN_FLOP_PER_UTT / (ms * 1e-3) / 1e12     # per GPU
     rec = {"metric": "utterances/sec through the triplet training step (3 forwards + loss + backward + allreduce + Adagrad)",
            "value": utt_per_step / (ms * 1e-3), "unit": "utt/s", "n_gpus": world, "steps": K, "warmup": W,
-           "ms_per_step": ms, "windows": {"n": len(ws), "ms_per_step_min": min(ws) / K, "ms_per_step_max": max(ws) / K,
-                                            "ms_per_step_each": [round(w / K, 4) for w in ws]},
-           "higher_is_better": True, "scaling": "weak", "dtype": args.dtype,
+           "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "dtype": args.dtype,
            "config": {"workload": f"triplet training step, batch {B} triplets per GPU (anchor/pos/neg), synthetic 64x{T} fbank, "
                                   f"branch A (train_triplet.py:215-224), Adagrad lr 0.1 (BASELINE configs[{2 if world == 1 else 4}])",
                       "global_batch_triplets": B * world,
@@ -747,7 +788,13 @@ def main():
     ap.add_argument("--workload", default="all", choices=["all", "infer", "train", "allpairs"],
                     help="all (default): the headline line (batch-64 embedding inference, BASELINE configs[1]) carrying "
                          "`train` (configs[2]/[4]) and `allpairs` (configs[3]) sub-records; infer/train/allpairs: that workload alone")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what each workload's last timed step computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the outputs of our arm; --impl reference times a shrinking sample of the batch")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -777,24 +824,27 @@ def main():
         dist.init_process_group("nccl", device_id=D.dev)
 
     line = None
+    outputs = {}
     if args.workload in ("all", "infer"):
-        line = bench_infer(args, D)
+        line = bench_infer(args, D, outputs)
     if args.workload in ("all", "train"):
-        rec = bench_train(args, D)
+        rec = bench_train(args, D, outputs)
         if rank == 0:
             if line is None:
                 line = dict(rec, vs_baseline=None, data="synthetic")
             else:
                 line["train"] = rec
     if args.workload == "all" and world == 1:
-        line["other_operand_dtype"] = bench_other_dtype(args, D)
+        line["other_operand_dtype"] = bench_other_dtype(args, D, outputs)
     if args.workload in ("all", "allpairs") and rank == 0:
-        rec = bench_allpairs(args, D)
+        rec = bench_allpairs(args, D, outputs)
         if line is None:
             line = dict(rec, n_gpus=1, ms_per_step=rec["value"] / 1e3, scaling="weak", vs_baseline=None, data="synthetic",
                         e2e={"value": rec["value"], "unit": "us", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0})
         else:
             line["allpairs"] = rec
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         emit(line)
     if world > 1:
